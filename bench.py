@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PGPE generations/s on synthetic Rastrigin (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--popsize P] [--dim D]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--popsize P] [--dim D] [--dump-outputs DIR]
 
 Workload (config.workload): PGPE (symmetric sampling, ClipUp, centered ranking, stdev_max_change 0.2; the reference's
 defaults), Rastrigin, popsize 1,000,000 x dim 10,000 fp32 -- the configuration BASELINE.json's metric is quoted on; the
@@ -66,7 +66,12 @@ def parse_args():
     ap.add_argument("--no-sharded-parity", action="store_true", help="skip the sharded-vs-unsharded parity leg at N > 1")
     ap.add_argument("--cuda-graph", type=int, default=-1, help="1/0: replay each generation from a CUDA graph. Default: 0 at N = 1 (kernels are timed live inside the timed region), 1 at N > 1 (the fused kernel is then timed stand-alone right after the timed region)")
     ap.add_argument("--peer", type=int, default=-1, help="1/0: at N > 1 move fitnesses and gradients between the GPUs from inside the producing kernels (NVLink peer memory, evotorch_b200/peer.py) instead of NCCL all_gather/all_reduce. Default: 1 at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last timed generation "
+                    "computed as DIR/<name>.npy: center, stdev, mean_eval, the fitnesses and a fixed, seeded sample of population rows "
+                    "(at most 64 MB in all); inputs are seeded, so two builds can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     cfg = CONFIGS[a.config]
     a.popsize = cfg["popsize"] if a.popsize is None else a.popsize
     a.dim = cfg["dim"] if a.dim is None else a.dim
@@ -335,6 +340,8 @@ def run_ours(args):
     clock_info = clocks.stop(t_begin, t_end) if clocks is not None else None
     mean_eval = float(searcher.status["mean_eval"])
     value = K / (elapsed_ms / 1e3)
+    if args.dump_outputs and rank == 0:  # before anything below launches into the population's buffers
+        dump_outputs(searcher, args.dump_outputs)
 
     # ---- roofline of the dominant kernel (fused sample + evaluate): algorithmic bytes = the population written once
     n_local = N // world
@@ -474,6 +481,37 @@ def run_ours(args):
                                                  with_gpu_eager=True)
     emit(line)
     finish()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(searcher, directory: str) -> None:
+    """What a caller of `searcher.step()` receives after the last step, as float32 / float64 .npy files: the distribution's
+    center and stdev, mean_eval, and, where this process holds the population, its fitnesses and a sample of its rows.
+    Samples are drawn with a fixed seed so that they name the same rows in every run; together they stay within DUMP_BYTES."""
+    import numpy as np
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    status = searcher.status
+    out = {"center": status["center"], "stdev": status["stdev"], "mean_eval": np.float64(status["mean_eval"])}
+    pop = searcher.population  # None when the population is row-sharded over ranks
+    if pop is not None:
+        n, d = len(pop), pop.solution_length
+        budget = (DUMP_BYTES - 8 * d - 64) // 4  # float32 elements left after center, stdev and mean_eval
+        gen = torch.Generator().manual_seed(SEED)
+        fitness = pop.evals[:, searcher.obj_index]
+        n_fit = min(n, budget // 2)
+        if n_fit < n:
+            fitness = fitness[torch.randperm(n, generator=gen)[:n_fit].sort().values.to(fitness.device)]
+        out["fitness"] = fitness
+        n_rows = min(n, 512, max(1, (budget - n_fit) // d))
+        rows = torch.randperm(n, generator=gen)[:n_rows].sort().values.tolist()
+        out["population_rows"] = torch.stack([pop[i].values for i in rows])  # row by row: a lazy population regenerates them
+    for name, value in out.items():
+        arr = value.detach().float().cpu().numpy() if isinstance(value, torch.Tensor) else np.asarray(value)
+        np.save(os.path.join(directory, f"{name}.npy"), arr)
 
 
 def sharded_parity_leg(dev, use_peer: bool) -> dict:

@@ -321,6 +321,62 @@ def test_bench_reference_arm_prints_one_json_line():
     assert abs(1.0 / lin["extrapolated_s_per_generation"] - d["value"]) < 1e-9 * d["value"] and d["cpu_baseline"]["extrapolated"] is True
 
 
+def _load_dir(path):
+    return {f[:-4]: np.load(os.path.join(path, f)) for f in sorted(os.listdir(path))}
+
+
+def test_bench_dump_outputs_are_float_bounded_and_seeded(tmp_path, monkeypatch):
+    import bench
+    from evotorch_b200 import objectives
+
+    def run():
+        s = PGPE(Problem("min", objectives.rastrigin, initial_bounds=(-5.12, 5.12), solution_length=40, device="cpu", seed=0), popsize=600,
+                 center_learning_rate=0.5, stdev_learning_rate=0.1, stdev_init=1.0)
+        s.run(3)
+        return s
+
+    s = run()
+    bench.dump_outputs(s, str(tmp_path / "a"))
+    bench.dump_outputs(run(), str(tmp_path / "b"))
+    a, b = _load_dir(tmp_path / "a"), _load_dir(tmp_path / "b")
+    assert sorted(a) == ["center", "fitness", "mean_eval", "population_rows", "stdev"]
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64), name
+        np.testing.assert_array_equal(a[name], b[name], err_msg=name)
+    np.testing.assert_array_equal(a["center"], s.status["center"].numpy())
+    np.testing.assert_array_equal(a["fitness"], s.population.evals[:, 0].numpy())
+    X = s.population.values.numpy()
+    assert a["population_rows"].shape == (512, 40) and all((X == r).all(1).any() for r in a["population_rows"])
+    # a smaller budget samples the fitnesses and rows instead of exceeding it
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    bench.dump_outputs(s, str(tmp_path / "c"))
+    c = _load_dir(tmp_path / "c")
+    assert sum(v.nbytes for v in c.values()) <= 4000 and 0 < len(c["fitness"]) < 600 and len(c["population_rows"]) >= 1
+    assert np.isin(c["fitness"], a["fitness"]).all()
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_of_the_timed_path(tmp_path):
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for tag in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--popsize", "20000", "--dim",
+                            "1000", "--no-cpu-baseline", "--no-e2e", "--no-other-configs", "--dump-outputs", str(tmp_path / tag)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        dumps.append(_load_dir(tmp_path / tag))
+    a, b = dumps
+    assert sorted(a) == ["center", "fitness", "mean_eval", "population_rows", "stdev"]
+    assert a["fitness"].shape == (20000,) and a["population_rows"].shape == (512, 1000) and a["center"].shape == (1000,)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for name in a:
+        assert a[name].dtype in (np.float32, np.float64) and np.isfinite(a[name]).all(), name
+        np.testing.assert_allclose(a[name], b[name], rtol=1e-6, atol=1e-6, err_msg=name)
+
+
 # ------------------------------------------------------------------------------------------------ pickling / checkpoints (SURVEY 8 f4)
 def test_pickling_logger_files_items_and_resume(tmp_path, capsys):
     import pickle

@@ -1,27 +1,30 @@
-"""In the build container (where /root/reference exists) run a few of the REFERENCE's own unit-test files against this package
-through scripts/run_reference_tests.py (`import evotorch` resolves to `evotorch_b200`; nothing is copied).  Skipped anywhere
-else -- in particular on the GPU box.  The full list and its results: profiles/r01_reference_unit_tests.txt."""
+"""The public helpers that the reference's own unit tests cover (hooks, ranking, the optimizer classes, read-only tensors,
+the decorators, `expects_ndim` / `rowwise`, the functional optimizers) must behave as the reference does: every
+observation of tests/golden/reference_api_probe.py on this package equals the reference's, stored in
+tests/golden/reference_api_golden.npz by tests/golden/gen_reference_api_golden.py."""
 
 import os
-import re
-import subprocess
 import sys
 
+import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TESTS = "/root/reference/tests"
+HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.join(HERE, "golden"))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="the reference checkout is only present in the build container")
+from reference_api_probe import GROUPS, probe  # noqa: E402
 
 
-@pytest.mark.parametrize("files,min_passed", [
-    (["test_hook.py", "test_ranking.py", "test_optimizers.py", "test_read_only_tensor.py"], 22),
-    (["test_decorators.py", "test_expects_ndim.py", "test_func_alg.py"], 54),
-])
-def test_reference_unit_tests_pass_against_this_package(files, min_passed):
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "run_reference_tests.py"), *files], capture_output=True, text=True,
-                         cwd=ROOT, timeout=300).stdout
-    summary = out.strip().splitlines()[-1]
-    assert "failed" not in summary and "error" not in summary, out[-3000:]
-    assert int(re.search(r"(\d+) passed", summary).group(1)) >= min_passed, summary
+@pytest.mark.parametrize("group", GROUPS)
+def test_public_helpers_match_reference(group):
+    with np.load(os.path.join(HERE, "golden", "reference_api_golden.npz")) as z:
+        expected = {k[len(group) + 1:]: z[k] for k in z.files if k.startswith(group + "/")}
+    got = probe("evotorch_b200", group)
+    assert sorted(got) == sorted(expected)
+    for key, want in expected.items():
+        have = np.asarray(got[key])
+        assert have.shape == want.shape, key
+        if want.dtype.kind in "fc":
+            np.testing.assert_allclose(have, want, rtol=1e-6, atol=1e-6, err_msg=key)
+        else:
+            np.testing.assert_array_equal(have, want, err_msg=key)
