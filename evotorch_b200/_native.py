@@ -60,9 +60,6 @@ _SIGNATURES = {
                                       c_size_t, _P]),
     "evok_mlp_forward_shared_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, _P]),
     "evok_mlp_forward_shared": (c_int, [_P, c_int64, c_int64, _P, c_int64, c_int64, c_int, _P, _P, _P, _P, c_size_t, _P]),
-    "evok_gemm_gather_rows": (c_int, [_P, c_int64, c_int64, c_int64, c_int64, _P, c_int64, c_int64, c_int64, c_int64, c_int, _P, c_int64, _P]),
-    "evok_gemm_gather_rows_workspace_bytes": (c_size_t, [c_int64, c_int64]),
-    "evok_gemm_gather_rows_ws": (c_int, [_P, c_int64, c_int64, c_int64, c_int64, _P, c_int64, c_int64, c_int64, c_int64, c_int, _P, c_int64, c_int, _P, c_size_t, _P]),
     "evok_gemm_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64]),
     "evok_gemm_nt": (c_int, [_P, c_int64, _P, c_int64, c_int64, c_int64, c_int64, _P, c_int64, _P, c_int64, _P, _P, _P, c_size_t, _P]),
     "evok_gemm_nt_affine": (c_int, [_P, c_int64, _P, c_int64, c_int64, c_int64, c_int64, _P, c_int64, _P, _P, c_int64, _P, _P, c_size_t, _P]),
@@ -72,8 +69,6 @@ _SIGNATURES = {
     "evok_peer_open": (c_int, [_P, _P]),
     "evok_peer_close": (c_int, [_P]),
     "evok_peer_free": (c_int, [_P]),
-    "evok_sample_eval_push": (c_int, [c_int, _P, c_int64, _P, _P, c_int64, c_int64, c_int64, c_int, c_uint64, c_uint64, _P, c_int, c_int, _P, _P,
-                                      _P, _P, _P]),
     "evok_peer_push": (c_int, [_P, c_int64, c_int64, c_int, c_int, _P, _P, _P, _P]),
     "evok_peer_wait": (c_int, [_P, c_int, _P, _P, c_uint64, _P]),
     "evok_grad_push": (c_int, [c_int, _P, c_int64, _P, _P, _P, c_int64, c_int64, c_int64, c_uint64, c_uint64, _P, c_float, c_float, c_int, c_int,

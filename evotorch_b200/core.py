@@ -515,7 +515,7 @@ class Problem(Clonable):
         return {"best": self._best, "worst": self._worst}
 
     # ------------------------------------------------------------------ pickling (core.py:2711-2734)
-    _TRANSIENT = ("_peer_exchange", "_active_peer", "_grad_batches", "_grad_scratch", "_d2h_stage")
+    _TRANSIENT = ("_peer_exchange", "_grad_batches", "_grad_scratch", "_d2h_stage")
 
     def __getstate__(self) -> dict:
         """Device-mapped and cached objects (peer-exchange buffers, gradient batches, the CUDA-graph generation counter) are
@@ -545,13 +545,8 @@ class Problem(Clonable):
             # the hook runs AFTER the new population is defined (core.py:2559 of the reference calls it inside evaluate(), after
             # distribution.sample): `batch.values` regenerates the new samples from the recipe.  A lazy batch is read-only.
             self._before_eval_hook(batch)
-            peer = getattr(self, "_active_peer", None)
-            if peer is not None:  # sharded generation over NVLink peer memory: the fitness all-gather happens inside the kernel
-                ops.sample_eval_push(obj, None, mu, sigma, n_rows=n, symmetric=distribution.SYMMETRIC, seed=seed, stream_id=stream_id,
-                                     row0=self.philox_row0, peer=peer, stream_offset=self.philox_stream_offset)
-            else:
-                ops.sample_eval(obj, None, mu, sigma, n_rows=n, symmetric=distribution.SYMMETRIC, seed=seed, stream_id=stream_id,
-                                row0=self.philox_row0, f=batch._evdata.view(-1), stream_offset=self.philox_stream_offset)
+            ops.sample_eval(obj, None, mu, sigma, n_rows=n, symmetric=distribution.SYMMETRIC, seed=seed, stream_id=stream_id,
+                            row0=self.philox_row0, f=batch._evdata.view(-1), stream_offset=self.philox_stream_offset)
             self._finish_evaluation(batch)
             return
         values = batch.access_values()
@@ -571,13 +566,6 @@ class Problem(Clonable):
         evdata = batch._evdata
         direct = evdata.shape[1] == 1 and evdata.dtype == torch.float32 and evdata.is_contiguous()
         f = evdata.view(-1) if direct else torch.empty(n, dtype=torch.float32, device=values.device)
-        peer = getattr(self, "_active_peer", None)
-        if peer is not None:  # sharded generation over NVLink peer memory (evdata IS this rank's slice of peer.f_all)
-            ops.sample_eval_push(obj, values, distribution.mu.contiguous(), distribution.sigma.contiguous(), n_rows=n,
-                                 symmetric=distribution.SYMMETRIC, seed=seed, stream_id=stream_id, row0=self.philox_row0, peer=peer,
-                                 stream_offset=self.philox_stream_offset)
-            self._finish_evaluation(batch)
-            return
         ops.sample_eval(obj, values, distribution.mu.contiguous(), distribution.sigma.contiguous(), n_rows=n,
                         symmetric=distribution.SYMMETRIC, seed=seed, stream_id=stream_id, row0=self.philox_row0, f=f,
                         stream_offset=self.philox_stream_offset)

@@ -271,4 +271,12 @@ __device__ __forceinline__ float activate_fast(float v, int act) {
   }
 }
 
+// Stacked-rows GEMM of the shared-minibatch policy forward (evok_gemm.cu, used by evok_mlp.cu):
+//   C[(i * n_cols + b) * rows_per_batch + h] = act( sum_k W_i[h, k] * X[b, k] + bias_i[h] )
+// W_i = params + i * batch_stride + w_offset (rows_per_batch x K, row-major, any 4-byte alignment), bias_i = params + i * batch_stride +
+// bias_offset (bias_offset < 0: none); X is n_cols x K at pitch ldx.  ws: gemm_gather_rows_workspace_bytes(n_cols, K) bytes.
+size_t gemm_gather_rows_workspace_bytes(int64_t n_cols, int64_t K);
+int gemm_gather_rows_ws(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch, int64_t n_batches, const float* X,
+                        int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset, int act, float* C, void* ws, size_t ws_bytes, void* stream);
+
 }  // namespace evok

@@ -162,6 +162,7 @@ __device__ __forceinline__ void split_lo_tile(uint32_t src, uint32_t dst) {
   }
 }
 
+// parameters of the generic kernel (gemm_tf32x3_kernel)
 struct GemmParams {
   int M, N, K;
   int kblocks_per_split;
@@ -178,17 +179,22 @@ struct GemmParams {
   const float* affine_E;
   int64_t lde;
   const float* affine_u;
-  // GATHER (batched policy forward, stacked weight rows): row m of the A operand lives at
-  //   gather_a + (m / ga_rows_per_batch) * ga_batch_stride + (m % ga_rows_per_batch) * ga_row_stride     (any 4-byte alignment)
-  // and the epilogue applies  C = act(acc + row_bias[(m / rows_per_batch) * rb_batch_stride + m % rows_per_batch])
+  long long* trace;  // -DEVOK_GEMM_TRACE builds only: clock64() stamps of CTA 0's roles per K-block (scripts/gemm_trace.py)
+};
+
+// parameters of the persistent gather kernel (gemm_gather_persistent_kernel, batched policy forward, stacked weight rows): row m of
+// the A operand lives at
+//   gather_a + (m / ga_rows_per_batch) * ga_batch_stride + (m % ga_rows_per_batch) * ga_row_stride     (any 4-byte alignment)
+// and the epilogue applies  act(acc + row_bias[(m / rows_per_batch) * rb_batch_stride + m % rows_per_batch])  and stores it unit-fastest:
+//   C[(batch * N + col) * rows_per_batch + row_in_batch]     (one cache line per store instruction)
+struct GatherParams {
+  int M, N, K;
+  float* C;
   const float* gather_a;
   int64_t ga_rows_per_batch, ga_batch_stride, ga_row_stride;
   const float* row_bias;
   int64_t rb_batch_stride;
   int row_act;
-  int debug;  // measurement only (EVOK_GATHER_DEBUG): 1 = skip the global loads of the gather, 2 = skip bias / activation
-  int b_lo_tma;  // CONVERT: the lo tile of B comes from a pre-split copy (map_b_lo) instead of being derived by the converter warps
-  int c_unit_fastest;  // persistent gather kernel: C[(batch * N + col) * rows_per_batch + row_in_batch] (one cache line per store instruction)
   long long* trace;  // -DEVOK_GEMM_TRACE builds only: clock64() stamps of CTA 0's roles per K-block (scripts/gather_trace.py)
 };
 
@@ -209,19 +215,7 @@ struct GemmParams {
 // register accumulators with ordinary round-to-nearest fp32 adds while the MMA warp fills the other TMEM accumulator.
 constexpr int kGemmChunk = 4;
 
-__device__ __noinline__ float gemm_act(float v, int act) {
-  switch (act) {
-    case EVOK_ACT_TANH: return tanhf(v);
-    case EVOK_ACT_RELU: return fmaxf(v, 0.0f);
-    case EVOK_ACT_SIGMOID: return __fdiv_rn(1.0f, 1.0f + expf(-v));
-    default: return v;
-  }
-}
-
-// GATHER (implies CONVERT): the A operand is not TMA-addressable (rows only 4-byte aligned, non-uniform pitch: the stacked first-layer
-// weights of a population of flat parameter vectors); the two converter warps fetch its tile with coalesced 128-byte row loads and
-// write BOTH the raw and the lo tile in the 128-byte-swizzled layout the tensor core expects, so the weights are read from HBM once.
-template <bool CONVERT, bool GATHER = false>
+template <bool CONVERT>
 __global__ void __launch_bounds__(kGemmThreads, 1)
     gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                        const __grid_constant__ CUtensorMap map_b_hi, const __grid_constant__ CUtensorMap map_b_lo, const GemmParams p) {
@@ -270,12 +264,12 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
         bar_wait(&empty[s], (use & 1) ^ 1);  // first use of a stage passes immediately (tight poll: with two stages the wake-up is on the critical path)
         EVOK_TRACE(9, (uint32_t)i);
         unsigned char* st = base + (size_t)s * kStageBytes;
-        bar_expect_tx(&full[s], (GATHER ? kTileBBytes : (CONVERT ? kTileABytes + kTileBBytes : kStageBytes)) + ((CONVERT && p.b_lo_tma) ? kTileBBytes : 0u));
+        bar_expect_tx(&full[s], CONVERT ? kTileABytes + kTileBBytes : kStageBytes);
         const int kx = (kb_begin + i) * kGemmBK;
-        if (!GATHER) tma_load_2d(st, &map_a_hi, kx, m0, &full[s]);
+        tma_load_2d(st, &map_a_hi, kx, m0, &full[s]);
         if (!CONVERT) tma_load_2d(st + kTileABytes, &map_a_lo, kx, m0, &full[s]);
         tma_load_2d(st + 2 * kTileABytes, &map_b_hi, kx, n0, &full[s]);
-        if (!CONVERT || p.b_lo_tma) tma_load_2d(st + 2 * kTileABytes + kTileBBytes, &map_b_lo, kx, n0, &full[s]);
+        if (!CONVERT) tma_load_2d(st + 2 * kTileABytes + kTileBBytes, &map_b_lo, kx, n0, &full[s]);
       }
     }
   } else if (warp == 1) {
@@ -315,47 +309,10 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     // the tensor core (async proxy) and signal the MMA warp.  Runs one or two K-blocks ahead of the MMAs.
     if (CONVERT) {
       const int ct = threadIdx.x - 64;  // 0 .. 63
-      auto lo_of = [](float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); };
-      // GATHER: the A tile of K-block i is fetched with 4-byte cp.async copies (global -> shared, no registers, zero fill outside
-      // the matrix): one 128-byte row segment per warp instruction, 64 rows per warp, all in flight at once; element (r, k) of a
-      // 128B-swizzled K-major tile sits at  r * 128 + ((k / 4) ^ (r % 8)) * 16 + (k % 4) * 4.  The copy of block i + 1 is issued
-      // right after block i has been converted, so a 16 KB tile per SM is in flight while the tensor core works on block i.
-      auto issue_gather = [&](int i) {
-        const int s = i % kGemmStages;
-        const uint32_t use = i / kGemmStages;
-        bar_wait(&empty[s], (use & 1) ^ 1);  // the stage's previous MMAs are done
-        const uint32_t st_a = s32(base + (size_t)s * kStageBytes);
-        const int kcol = (kb_begin + i) * kGemmBK + lane;
-        const bool k_ok = kcol < p.K;
-        const int wrow0 = (warp - 2) * 64;
-        const int m_first = m0 + wrow0;
-        int hrow = m_first % (int)p.ga_rows_per_batch;
-        const float* rowp = p.gather_a + (int64_t)(m_first / (int)p.ga_rows_per_batch) * p.ga_batch_stride + (int64_t)hrow * p.ga_row_stride + kcol;
-        const int64_t wrap = p.ga_batch_stride - p.ga_rows_per_batch * p.ga_row_stride;
-#pragma unroll 8
-        for (int it = 0; it < 64; ++it) {
-          const int r = wrow0 + it;
-          const bool ok = k_ok && (m0 + r < p.M) && p.debug != 1;
-          const uint32_t off = (uint32_t)r * 128u + ((((uint32_t)lane >> 2) ^ ((uint32_t)r & 7u)) << 4) + (((uint32_t)lane & 3u) << 2);
-          const float* src = ok ? rowp : p.gather_a;  // a valid address even when nothing is read (src-size 0 -> zero fill)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(st_a + off), "l"(src), "r"(ok ? 4 : 0) : "memory");
-          rowp += p.ga_row_stride;
-          if (++hrow == (int)p.ga_rows_per_batch) {
-            hrow = 0;
-            rowp += wrap;
-          }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-      };
-      if (GATHER && num_kb > 0) issue_gather(0);
       for (int i = 0; i < num_kb; ++i) {
         const int s = i % kGemmStages;
         const uint32_t use = i / kGemmStages;
         unsigned char* st = base + (size_t)s * kStageBytes;
-        if (GATHER) {
-          asm volatile("cp.async.wait_group 0;" ::: "memory");  // this thread's copies of block i have landed
-          asm volatile("bar.sync 1, 64;" ::: "memory");         // ... and so have the other converter warp's
-        }
         if (threadIdx.x == 64) EVOK_TRACE(0, (uint32_t)i);
         bar_wait(&full[s], use & 1);
         if (threadIdx.x == 64) EVOK_TRACE(1, (uint32_t)i);
@@ -364,16 +321,13 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
         const float4* b_raw = reinterpret_cast<const float4*>(st + 2 * kTileABytes);
         float4* b_lo = reinterpret_cast<float4*>(st + 2 * kTileABytes + kTileBBytes);
         // (a single warp runs this dependent stream at ~0.2 IPC, so the instruction count per K-block is what matters: shared-space
-        // 16-byte loads / stores with immediate offsets, 16 loads in flight; B is skipped when its lo tile came by TMA)
+        // 16-byte loads / stores with immediate offsets, 16 loads in flight)
         split_lo_tile<kTileABytes>(s32(a_raw) + (uint32_t)ct * 16u, s32(a_lo) + (uint32_t)ct * 16u);
-        if (!p.b_lo_tma) split_lo_tile<kTileBBytes>(s32(b_raw) + (uint32_t)ct * 16u, s32(b_lo) + (uint32_t)ct * 16u);
+        split_lo_tile<kTileBBytes>(s32(b_raw) + (uint32_t)ct * 16u, s32(b_lo) + (uint32_t)ct * 16u);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy stores -> visible to the tensor core's reads
         __syncwarp();
         if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s32(&conv[s])) : "memory");
         if (threadIdx.x == 64) EVOK_TRACE(3, (uint32_t)i);
-        // the next block's copy is issued AFTER this block has been handed to the tensor core (its stage frees up when the MMAs of
-        // block i - 1 retire, which overlaps with the MMAs of block i)
-        if (GATHER && i + 1 < num_kb) issue_gather(i + 1);
       }
     }
   } else {
@@ -404,25 +358,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     };
     for (int ch = 0; ch < num_chunks; ++ch) fold_chunk(ch);
     if (threadIdx.x == 128) EVOK_TRACE(13, 1u);  // all chunks folded: the store phase starts
-    if (GATHER && p.row_bias && p.debug != 2) {  // C = act(acc + bias of this row): TMEM lane = row of the tile
-      const int64_t m = (int64_t)m0 + quad * 32 + lane;
-      if (m < p.M) {
-        const int64_t bi = m / p.ga_rows_per_batch;
-        const float b = __ldg(p.row_bias + bi * p.rb_batch_stride + (m - bi * p.ga_rows_per_batch));
-        // the activation switch is hoisted out of the unrolled loop: one 128-fold copy of ONE activation per branch, the common
-        // NONE case is a plain add (a per-element switch with an inlined tanhf was 15 k instructions: instruction-cache bound)
-        if (p.row_act == EVOK_ACT_NONE) {
-#pragma unroll
-          for (int j = 0; j < kGemmBN / 2; ++j) acc[j] += b;
-        } else if (p.row_act == EVOK_ACT_RELU) {
-#pragma unroll
-          for (int j = 0; j < kGemmBN / 2; ++j) acc[j] = fmaxf(acc[j] + b, 0.0f);
-        } else {
-#pragma unroll
-          for (int j = 0; j < kGemmBN / 2; ++j) acc[j] = gemm_act(acc[j] + b, p.row_act);  // 128 calls of the out-of-line function
-        }
-      }
-    }
     // all MMAs have completed (the last tmem_full has fired), so the pipeline stages are free: use them as transpose scratch
     float* stile = reinterpret_cast<float*>(base) + (size_t)(warp - 4) * (32 * kEpiPitch);
     const float alpha = (p.C2 && p.alpha_dev) ? *p.alpha_dev : 1.0f;
@@ -478,8 +413,10 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
 }
 
 // ---- persistent gather GEMM (batched policy forward on ONE shared minibatch) ------------------------------------------------
-// Same arithmetic as gemm_tf32x3_kernel<true, true>, restructured for the shape this path has -- millions of A rows (the stacked
-// first-layer weights), a small B operand (the minibatch) that every tile re-reads:
+// Same arithmetic as gemm_tf32x3_kernel, for an A operand that is not TMA-addressable (rows only 4-byte aligned, non-uniform pitch: the
+// stacked first-layer weights of a population of flat parameter vectors, GatherParams): the two converter warps fetch its tile with
+// cp.async row copies and write BOTH the raw and the lo tile in the 128-byte-swizzled layout the tensor core expects, so the weights are
+// read from HBM once.  Built for the shape this path has -- millions of A rows, a small B operand (the minibatch) that every tile re-reads:
 //   * PERSISTENT: one CTA per SM walks the output tiles (tile = blockIdx.x + q * gridDim.x), so barrier set-up and the TMEM allocation
 //     happen once, and the epilogue of tile q (bias, activation, 128 KB of stores) runs while the tensor core is already two
 //     accumulator chunks into tile q + 1 (the two TMEM accumulators of the chunked accumulation double as the overlap buffer);
@@ -488,7 +425,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
 //   * the gathered A tiles live in a 4-deep ring of raw tiles (three 16 KB gathers in flight per SM while one is converted) with only
 //     two lo buffers behind it (a lo tile is derived right before its MMAs); the minibatch tiles (2 stages of hi + lo, 128 KB) come
 //     from L2;
-//   * the epilogue warps store their rows straight from registers (a row of the tile = 128 consecutive floats per thread).
+//   * the epilogue warps store straight from registers, unit-fastest (GatherParams): the 32 lanes of a warp, consecutive rows of one
+//     batch, write 128 consecutive bytes per store instruction.
 // the minibatch operand, pre-split into hi / lo and stored four times, copy s shifted right by s floats (xs[b][k'] = x[b][k' - s], zero
 // outside): TMA needs 16-byte aligned box coordinates (an odd K coordinate is an illegal instruction), so a tile whose rows sit sh
 // floats past a 16-byte boundary reads copy sh at the aligned coordinate 32 i instead of the original at 32 i - sh
@@ -508,7 +446,7 @@ constexpr size_t kPersSmemBytes =
     (size_t)(kPersRawStages + kPersLoStages) * kTileABytes + (size_t)kPersBStages * kPersBStageBytes + 1024 /*align*/ + 256;
 
 __global__ void __launch_bounds__(kGemmThreads, 1)
-    gemm_gather_persistent_kernel(const __grid_constant__ GatherMaps maps, const GemmParams p) {
+    gemm_gather_persistent_kernel(const __grid_constant__ GatherMaps maps, const GatherParams p) {
   extern __shared__ unsigned char gemm_smem_raw[];
   unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(gemm_smem_raw) + 1023) & ~(uintptr_t)1023);
   unsigned char* raw_base = base;                                             // gathered A tiles (= the hi operand)
@@ -581,10 +519,9 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
           bar_wait(&empty_b[s], ((g / kPersBStages) & 1) ^ 1);  // tight poll: the minibatch tile of block g + 2 is needed ~1 block later
           EVOK_TRACE(9, g);
           unsigned char* st = b_base + (size_t)s * kPersBStageBytes;
-          // (p.debug == 3, measurement only: the lo tile of the minibatch is not loaded -- wrong results, half the L2 -> SM traffic)
-          bar_expect_tx(&full_b[s], p.debug == 3 ? kTileBBytes : kPersBStageBytes);
+          bar_expect_tx(&full_b[s], kPersBStageBytes);
           tma_load_2d(st, &maps.hi[sh], i * kGemmBK, n0, &full_b[s]);
-          if (p.debug != 3) tma_load_2d(st + kTileBBytes, &maps.lo[sh], i * kGemmBK, n0, &full_b[s]);
+          tma_load_2d(st + kTileBBytes, &maps.lo[sh], i * kGemmBK, n0, &full_b[s]);
         }
       }
     }
@@ -759,7 +696,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
   } else {
     // ===== 8 epilogue warps: TMEM lane quadrant = warp % 4 (tile row = quadrant * 32 + lane), column half = (warp - 4) / 4 =====
     const int quad = warp & 3, half = (warp - 4) >> 2;
-    const bool vec_ok = ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0) && (p.ldc % 4 == 0);
     uint32_t gch = 0;
     for (int64_t q = 0; q < my_tiles; ++q) {
       const int64_t t = blockIdx.x + q * gridDim.x;
@@ -794,26 +730,23 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
         }
         // bias + activation applied four values at a time on the way out; one unrolled copy of the store loop per activation (a
         // per-element switch would not fit the instruction cache)
-        float* crow = p.C + m * p.ldc;
         const int col0 = n0 + half * (kGemmBN / 2);
         // unit-fastest layout: the 32 lanes of a warp (consecutive rows of one batch) write 128 consecutive bytes per instruction
         const int64_t bi_c = m / p.ga_rows_per_batch;
         float* ccol = p.C + (bi_c * p.N + col0) * p.ga_rows_per_batch + (m - bi_c * p.ga_rows_per_batch);
         const int64_t cstride = p.ga_rows_per_batch;
+        // (the full-width case stores unconditionally: with only per-element guards the compiler moves each activation under its
+        // own branch and the four no longer overlap -- measured 2 % slower over the whole forward)
         auto store4 = [&](int j, float v0, float v1, float v2, float v3) {
           const int col = col0 + j;
-          if (p.c_unit_fastest) {
-            const float v[4] = {v0, v1, v2, v3};
+          const float v[4] = {v0, v1, v2, v3};
+          if (col + 4 <= p.N) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) ccol[(int64_t)(j + u) * cstride] = v[u];
+          } else {
 #pragma unroll
             for (int u = 0; u < 4; ++u)
               if (col + u < p.N) ccol[(int64_t)(j + u) * cstride] = v[u];
-          } else if (vec_ok && col + 4 <= p.N) {
-            *reinterpret_cast<float4*>(crow + col) = make_float4(v0, v1, v2, v3);
-          } else {
-            const float v[4] = {v0, v1, v2, v3};
-#pragma unroll
-            for (int u = 0; u < 4; ++u)
-              if (col + u < p.N) crow[col + u] = v[u];
           }
         };
         if (p.row_act == EVOK_ACT_NONE) {
@@ -854,16 +787,6 @@ __global__ void __launch_bounds__(256) split_tf32_kernel(const float* __restrict
   const float h = __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
   hi[r * ldo + c] = h;
   lo[r * ldo + c] = v - h;
-}
-
-// lo[r][c] = x[r][c] - trunc_tf32(x[r][c])   (the pre-split lo copy of the B operand, pitch ldo)
-__global__ void __launch_bounds__(256) lo_tf32_kernel(const float* __restrict__ x, int64_t ldx, int64_t rows, int64_t cols, float* __restrict__ lo,
-                                                      int64_t ldo) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= rows * ldo) return;
-  const int64_t r = i / ldo, c = i - r * ldo;
-  const float v = c < cols ? x[r * ldx + c] : 0.0f;
-  lo[i] = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
 }
 
 // the four shifted hi / lo copies of the minibatch (GatherMaps): hi[s][r][c] / lo[s][r][c] of x[r][c - s], zero for c - s outside [0, cols)
@@ -1024,18 +947,7 @@ static int gemm_impl(const float* A, int64_t lda, const float* B, int64_t ldb, i
   float* partial = (float*)(w8 + g.off_partial);
   // Operands that TMA can address directly (16-byte aligned base and pitch: every matrix this package allocates) are read from
   // HBM once, by the GEMM itself, which derives the lo halves in shared memory; otherwise a pre-pass writes aligned split copies.
-  static const int allow_convert = [] {
-    const char* e = getenv("EVOK_GEMM_CONVERT");
-    return e ? atoi(e) : 1;
-  }();
-  const bool convert = allow_convert && tma_ok(A, lda) && tma_ok(B, ldb);
-  static const int allow_b_lo = [] {
-    // =1: B's lo tile by TMA from a pre-split copy instead of the converter warps.  Measured: 8192^3 4.94 vs 5.05 ms, but 52 vs 44 us at
-    // the CMA-ES sizes (the extra pre-pass launch), and the K loop is bound by the 2-stage load latency either way -- off by default
-    const char* e = getenv("EVOK_GEMM_B_LO_TMA");
-    return e ? atoi(e) : 0;
-  }();
-  const bool b_lo_tma = convert && allow_b_lo;
+  const bool convert = tma_ok(A, lda) && tma_ok(B, ldb);
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
   int rc;
   if (convert) {
@@ -1043,12 +955,6 @@ static int gemm_impl(const float* A, int64_t lda, const float* B, int64_t ldb, i
     if ((rc = make_map(&mb_hi, B, N, K, ldb, kGemmBN))) return rc;
     ma_lo = ma_hi;
     mb_lo = mb_hi;
-    if (b_lo_tma) {  // B's lo tile by TMA from a pre-split copy: the converter warps only derive A's (a third of the element-wise work)
-      float* b_lo = (float*)(w8 + g.off_b_lo);
-      lo_tf32_kernel<<<(unsigned)((N * g.ldk + 255) / 256), 256, 0, st>>>(B, ldb, N, K, b_lo, g.ldk);
-      EVOK_CHECK_LAUNCH();
-      if ((rc = make_map(&mb_lo, b_lo, N, K, g.ldk, kGemmBN))) return rc;
-    }
   } else {
     float* a_hi = (float*)(w8 + g.off_a_hi);
     float* a_lo = (float*)(w8 + g.off_a_lo);
@@ -1077,12 +983,6 @@ static int gemm_impl(const float* A, int64_t lda, const float* B, int64_t ldb, i
   p.affine_E = aff ? aff->E : nullptr;
   p.lde = aff ? aff->lde : 0;
   p.affine_u = aff ? aff->u : nullptr;
-  p.gather_a = nullptr;
-  p.ga_rows_per_batch = p.ga_batch_stride = p.ga_row_stride = p.rb_batch_stride = 0;
-  p.row_bias = nullptr;
-  p.row_act = 0;
-  p.debug = 0;
-  p.b_lo_tma = b_lo_tma ? 1 : 0;
   p.trace = nullptr;
 #ifdef EVOK_GEMM_TRACE
   {
@@ -1092,15 +992,14 @@ static int gemm_impl(const float* A, int64_t lda, const float* B, int64_t ldb, i
 #endif
   static bool attr_set = false;
   if (!attr_set) {
-    if (cudaFuncSetAttribute(gemm_tf32x3_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(gemm_tf32x3_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(gemm_tf32x3_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess)
+    if (cudaFuncSetAttribute(gemm_tf32x3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess ||
+        cudaFuncSetAttribute(gemm_tf32x3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess)
       return (int)cudaGetLastError();
     attr_set = true;
   }
   dim3 grid((unsigned)((M + kGemmBM - 1) / kGemmBM), (unsigned)((N + kGemmBN - 1) / kGemmBN), (unsigned)g.splits);
-  if (convert) gemm_tf32x3_kernel<true, false><<<grid, kGemmThreads, kGemmSmemBytes, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
-  else gemm_tf32x3_kernel<false, false><<<grid, kGemmThreads, kGemmSmemBytes, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
+  if (convert) gemm_tf32x3_kernel<true><<<grid, kGemmThreads, kGemmSmemBytes, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
+  else gemm_tf32x3_kernel<false><<<grid, kGemmThreads, kGemmSmemBytes, st>>>(ma_hi, ma_lo, mb_hi, mb_lo, p);
   EVOK_CHECK_LAUNCH();
   if (split) {
     reduce_splits_kernel<<<(unsigned)((M * N + 255) / 256), 256, 0, st>>>(partial, g.splits, M * N, M, N, N, C, ldc, aff ? aff->k : nullptr,
@@ -1124,69 +1023,20 @@ extern "C" EVOK_API int evok_gemm_nt_affine(const float* A, int64_t lda, const f
   return gemm_impl(A, lda, B, ldb, M, N, K, C, ldc, nullptr, 0, nullptr, nullptr, &aff, ws, ws_bytes, stream);
 }
 
-// Stacked-rows GEMM of the batched policy forward:  C[(i, h), b] = act( sum_k W_i[h, k] * X[b, k] + bias_i[h] )
-// A rows gathered from the population matrix (see GemmParams::gather_a), B = the shared input batch X (n_cols x K, TMA: 16-byte aligned).
-extern "C" EVOK_API int evok_gemm_gather_rows(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch, int64_t n_batches,
-                                              const float* X, int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset, int act, float* C,
-                                              int64_t ldc, void* stream) {
-  if (!params || !X || !C) return EVOK_E_NULLPTR;
-  const int64_t M = rows_per_batch * n_batches;
-  if (rows_per_batch <= 0 || n_batches <= 0 || n_cols <= 0 || K <= 0 || ldx < K || ldc < n_cols || M >= (1ll << 31)) return EVOK_E_BADSIZE;
-  if (act < EVOK_ACT_NONE || act > EVOK_ACT_SIGMOID) return EVOK_E_BADENUM;
-  if (!tma_ok(X, ldx)) return EVOK_E_ALIGN;
-  CUtensorMap mb;
-  int rc;
-  if ((rc = make_map(&mb, X, n_cols, K, ldx, kGemmBN))) return rc;
-  GemmParams p{};
-  p.M = (int)M; p.N = (int)n_cols; p.K = (int)K;
-  p.kblocks_per_split = (int)((K + kGemmBK - 1) / kGemmBK);
-  p.C = C;
-  p.ldc = ldc;
-  p.gather_a = params + w_offset;
-  p.ga_rows_per_batch = rows_per_batch;
-  p.ga_batch_stride = batch_stride;
-  p.ga_row_stride = K;
-  p.row_bias = bias_offset >= 0 ? params + bias_offset : nullptr;
-  p.rb_batch_stride = batch_stride;
-  p.row_act = act;
-  {
-    const char* e = getenv("EVOK_GATHER_DEBUG");
-    p.debug = e ? atoi(e) : 0;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(gemm_tf32x3_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes) != cudaSuccess)
-      return (int)cudaGetLastError();
-    attr_set = true;
-  }
-  dim3 grid((unsigned)((M + kGemmBM - 1) / kGemmBM), (unsigned)((n_cols + kGemmBN - 1) / kGemmBN), 1);
-  gemm_tf32x3_kernel<true, true><<<grid, kGemmThreads, kGemmSmemBytes, (cudaStream_t)stream>>>(mb, mb, mb, mb, p);
-  EVOK_CHECK_LAUNCH();
-  return 0;
-}
-
-extern "C" EVOK_API size_t evok_gemm_gather_rows_workspace_bytes(int64_t n_cols, int64_t K) {
+// Stacked-rows GEMM of the batched policy forward (declared in evok_common.cuh) on the persistent kernel: X is split into four shifted
+// hi / lo copies in `ws` first, so any alignment / pitch of X is fine.
+size_t evok::gemm_gather_rows_workspace_bytes(int64_t n_cols, int64_t K) {
   if (n_cols <= 0 || K <= 0) return 512;
   return (size_t)8 * n_cols * round_up(K + 3, 4) * sizeof(float) + 512;  // 4 shifted copies of the hi and of the lo part
 }
 
-// The same product on the persistent kernel (gemm_gather_persistent_kernel): X is split into hi / lo copies in `ws` first (any
-// alignment / pitch of X is fine).  unit_fastest = 1 writes C[(batch * n_cols + col) * rows_per_batch + row] instead of the row-major
-// C[(batch * rows_per_batch + row) * ldc + col]: one cache line per store instruction of the epilogue instead of 32.
-// EVOK_GATHER_PERSISTENT=0 routes the row-major case to the one-tile-per-CTA kernel instead (measurement only).
-extern "C" EVOK_API int evok_gemm_gather_rows_ws(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch,
-                                                 int64_t n_batches, const float* X, int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset,
-                                                 int act, float* C, int64_t ldc, int unit_fastest, void* ws, size_t ws_bytes, void* stream) {
+int evok::gemm_gather_rows_ws(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch, int64_t n_batches,
+                              const float* X, int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset, int act, float* C, void* ws,
+                              size_t ws_bytes, void* stream) {
   if (!params || !X || !C || !ws) return EVOK_E_NULLPTR;
   const int64_t M = rows_per_batch * n_batches;
-  if (rows_per_batch <= 0 || n_batches <= 0 || n_cols <= 0 || K <= 0 || ldx < K || (!unit_fastest && ldc < n_cols) || M >= (1ll << 31))
-    return EVOK_E_BADSIZE;
+  if (rows_per_batch <= 0 || n_batches <= 0 || n_cols <= 0 || K <= 0 || ldx < K || M >= (1ll << 31)) return EVOK_E_BADSIZE;
   if (act < EVOK_ACT_NONE || act > EVOK_ACT_SIGMOID) return EVOK_E_BADENUM;
-  {
-    const char* e = getenv("EVOK_GATHER_PERSISTENT");
-    if (!unit_fastest && e && atoi(e) == 0 && tma_ok(X, ldx))
-      return evok_gemm_gather_rows(params, batch_stride, w_offset, rows_per_batch, n_batches, X, ldx, n_cols, K, bias_offset, act, C, ldc, stream);
-  }
   const int64_t ldk = round_up(K + 3, 4);
   char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
   if (ws_bytes < (size_t)(base - (char*)ws) + (size_t)8 * n_cols * ldk * sizeof(float)) return EVOK_E_WORKSPACE;
@@ -1200,11 +1050,9 @@ extern "C" EVOK_API int evok_gemm_gather_rows_ws(const float* params, int64_t ba
     if ((rc = make_map(&maps.hi[s], x_hi + s * n_cols * ldk, n_cols, ldk, ldk, kGemmBN))) return rc;
     if ((rc = make_map(&maps.lo[s], x_lo + s * n_cols * ldk, n_cols, ldk, ldk, kGemmBN))) return rc;
   }
-  GemmParams p{};
+  GatherParams p{};
   p.M = (int)M; p.N = (int)n_cols; p.K = (int)K;
-  p.kblocks_per_split = (int)((K + kGemmBK - 1) / kGemmBK);
   p.C = C;
-  p.ldc = ldc;
   p.gather_a = params + w_offset;
   p.ga_rows_per_batch = rows_per_batch;
   p.ga_batch_stride = batch_stride;
@@ -1212,11 +1060,6 @@ extern "C" EVOK_API int evok_gemm_gather_rows_ws(const float* params, int64_t ba
   p.row_bias = bias_offset >= 0 ? params + bias_offset : nullptr;
   p.rb_batch_stride = batch_stride;
   p.row_act = act;
-  p.c_unit_fastest = unit_fastest ? 1 : 0;
-  {
-    const char* e = getenv("EVOK_GATHER_DEBUG");
-    p.debug = e ? atoi(e) : 0;
-  }
 #ifdef EVOK_GEMM_TRACE
   {
     const char* e = getenv("EVOK_GATHER_TRACE_PTR");  // device pointer (hex) of a 512 x 16 int64 buffer

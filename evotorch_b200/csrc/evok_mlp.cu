@@ -170,7 +170,7 @@ __global__ void __launch_bounds__(kMlpThreads)
 }
 
 // ---- shared-minibatch forward (SupervisedNE with common_minibatch, supervisedne.py:337-347): layers 2..n of N networks on B samples.
-// The first layer is the tensor-core GEMM over the stacked weight rows (evok_gemm_gather_rows), which leaves
+// The first layer is the tensor-core GEMM over the stacked weight rows (gemm_gather_rows_ws), which leaves
 //   hid[(i * B + b) * H1 + h] = act_0(W_0^i x_b + b_0^i)[h]      (unit fastest: one cache line per store instruction of the GEMM epilogue);
 // this kernel takes one (network i, tile of 32 samples) per CTA, keeps the tile's activations in shared memory ([width][33]) and runs
 // the remaining layers with fp32 FMAs: thread = (sample lane, output neuron), the weight row is a broadcast load shared by the 32
@@ -394,7 +394,7 @@ extern "C" EVOK_API size_t evok_mlp_forward_shared_workspace_bytes(int64_t N, in
   if (chunk < 1) chunk = 1;
   if (chunk > 65535) chunk = 65535;
   if (chunk > N) chunk = N;
-  return (size_t)chunk * dims_host[1] * ldh * 4 + 256 + evok_gemm_gather_rows_workspace_bytes(B, dims_host[0]);
+  return (size_t)chunk * dims_host[1] * ldh * 4 + 256 + gemm_gather_rows_workspace_bytes(B, dims_host[0]);
 }
 
 // out[i, b, :] = net_i(X[b, :]) for N flat parameter rows and ONE shared input batch X (B x dims[0], 16-byte aligned rows).
@@ -430,7 +430,7 @@ extern "C" EVOK_API int evok_mlp_forward_shared(const float* params, int64_t ldp
   if (chunk > N) chunk = N;
   char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
   const size_t hid_bytes = ((size_t)chunk * h1 * ldh * 4 + 255) & ~(size_t)255;
-  const size_t gws_bytes = evok_gemm_gather_rows_workspace_bytes(B, spec.dims[0]);
+  const size_t gws_bytes = gemm_gather_rows_workspace_bytes(B, spec.dims[0]);
   if (ws_bytes < (size_t)(base - (char*)ws) + hid_bytes + gws_bytes) return EVOK_E_WORKSPACE;
   float* hid = reinterpret_cast<float*>(base);
   void* gws = base + hid_bytes;
@@ -453,8 +453,8 @@ extern "C" EVOK_API int evok_mlp_forward_shared(const float* params, int64_t ldp
   for (int64_t i0 = 0; i0 < N; i0 += chunk) {
     const int64_t c = (N - i0) < chunk ? (N - i0) : chunk;
     // layer 0 of the c networks as ONE stacked-rows tensor-core product: (c * H1 x in) * (in x B)
-    int rc = evok_gemm_gather_rows_ws(params + i0 * ldp, ldp, spec.w_off[0], h1, c, X, ldx, B, spec.dims[0],
-                                      spec.w_off[0] + (int64_t)spec.dims[0] * h1, spec.acts[0], hid, ldh, 1 /* unit fastest */, gws, gws_bytes, stream);
+    int rc = gemm_gather_rows_ws(params + i0 * ldp, ldp, spec.w_off[0], h1, c, X, ldx, B, spec.dims[0], spec.w_off[0] + (int64_t)spec.dims[0] * h1,
+                                 spec.acts[0], hid, gws, gws_bytes, stream);
     if (rc) return rc;
     const size_t smem2 = ((size_t)(h1 + 4) * kTail2Samples + (size_t)h1 * kTail2Groups * kTail2Slots + kTail2Groups * kTail2Slots + 128 * 2 * 8) * sizeof(float);
     if (n_layers == 2 && spec.dims[2] <= kTail2MaxOut && smem2 <= 200 * 1024 && (reinterpret_cast<uintptr_t>(hid) & 15) == 0 && h1 % 4 == 0) {

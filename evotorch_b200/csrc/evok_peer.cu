@@ -1,6 +1,6 @@
 // Peer exchange over NVLink / NVSwitch: buffer sharing between the per-GPU processes (CUDA IPC) and the two consumer-side
-// kernels -- the flag wait and the slot reduction.  The producer sides live in the kernels that produce the data
-// (sample_eval_kernel's fitness store, grad_finalize_push_kernel); see PeerSink / peer_signal_tail in evok_common.cuh.
+// kernels -- the flag wait and the slot reduction -- plus the fitness push.  The gradient's producer side lives in the kernel that
+// produces it (grad_finalize_push_kernel); see PeerSink / peer_signal_tail in evok_common.cuh.
 //
 // Protocol per exchange point (fitness gather, gradient reduce), all counters 64-bit and monotone:
 //   producer rank r, generation g : stores its data into every peer's buffer, fence.sys, flag[p][r] = g + 1 (st.release.sys)

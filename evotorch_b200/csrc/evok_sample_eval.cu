@@ -80,13 +80,11 @@ __device__ __forceinline__ void sample_group(const PhiloxKey& key, uint32_t sw, 
   }
 }
 
-// PUSH: the fitness of row i goes to row (row0 + i) of EVERY peer's fitness vector (the all-gather of the sharded
-// generation, fused into the producer) and the last CTA raises this rank's flag on every peer.
-template <int OBJ, bool SYM, bool STORE, bool VEC, bool PUSH>
+template <int OBJ, bool SYM, bool STORE, bool VEC>
 __global__ void __launch_bounds__(kSampleThreads, SampleTune<OBJ>::kMinBlocks)
     sample_eval_kernel(float* __restrict__ X, int64_t ldx, const float* __restrict__ mu, const float* __restrict__ sigma,
                        int64_t row0, int64_t n_units, int64_t D, const __grid_constant__ PhiloxKey key, const uint32_t* __restrict__ stream_off,
-                       float* __restrict__ f, const __grid_constant__ PeerSink sink, const unsigned long long* epoch, unsigned int* done) {
+                       float* __restrict__ f) {
   const int lane = threadIdx.x & 31;
   const uint32_t sw = key.stream_lo + (stream_off ? __ldg(stream_off) : 0u);
   const int64_t warps_total = (int64_t)gridDim.x * (kSampleThreads / 32);
@@ -116,20 +114,11 @@ __global__ void __launch_bounds__(kSampleThreads, SampleTune<OBJ>::kMinBlocks)
       float fm = 0.f;
       if (SYM) fm = accm.finish(D);
       if (lane == 0) {
-        if (PUSH) {
-          for (int p = 0; p < sink.world; ++p) {
-            float* fr = static_cast<float*>(sink.data[p]) + row0 + r;
-            fr[0] = fp;
-            if (SYM) fr[1] = fm;
-          }
-        } else {
-          f[r] = fp;
-          if (SYM) f[r + 1] = fm;
-        }
+        f[r] = fp;
+        if (SYM) f[r + 1] = fm;
       }
     }
   }
-  if (PUSH) peer_signal_tail(sink, epoch, done);
 }
 
 // Batched searches (functional ask/tell API with leading batch dimensions, funcpgpe.py:301-327): blockIdx.y = batch item, every
@@ -201,30 +190,19 @@ static int resident_grid(K kernel, int threads, int64_t units_per_cta_needed) {
   return (int)g;
 }
 
-struct PushArgs {
-  PeerSink sink;
-  const unsigned long long* epoch;
-  unsigned int* done;
-};
-
-template <int OBJ, bool SYM, bool STORE, bool PUSH = false>
+template <int OBJ, bool SYM, bool STORE>
 static int launch_sample(float* X, int64_t ldx, const float* mu, const float* sigma, int64_t row0, int64_t n_rows, int64_t D,
-                         uint64_t seed, uint64_t stream_id, const uint32_t* stream_off, float* f, cudaStream_t st,
-                         const PushArgs* push = nullptr) {
+                         uint64_t seed, uint64_t stream_id, const uint32_t* stream_off, float* f, cudaStream_t st) {
   const int64_t n_units = SYM ? n_rows / 2 : n_rows;
   const bool vec = (D % 4 == 0) && aligned16(mu) && aligned16(sigma) && (!STORE || (aligned16(X) && ldx % 4 == 0));
   const int64_t ctas_needed = (n_units + (kSampleThreads / 32) - 1) / (kSampleThreads / 32);
   const PhiloxKey key = make_philox_key(seed, stream_id);
-  PushArgs none{};
-  const PushArgs& pa = PUSH ? *push : none;
   if (vec) {
-    auto k = sample_eval_kernel<OBJ, SYM, STORE, true, PUSH>;
-    k<<<resident_grid(k, kSampleThreads, ctas_needed), kSampleThreads, 0, st>>>(X, ldx, mu, sigma, row0, n_units, D, key, stream_off, f, pa.sink,
-                                                                                pa.epoch, pa.done);
+    auto k = sample_eval_kernel<OBJ, SYM, STORE, true>;
+    k<<<resident_grid(k, kSampleThreads, ctas_needed), kSampleThreads, 0, st>>>(X, ldx, mu, sigma, row0, n_units, D, key, stream_off, f);
   } else {
-    auto k = sample_eval_kernel<OBJ, SYM, STORE, false, PUSH>;
-    k<<<resident_grid(k, kSampleThreads, ctas_needed), kSampleThreads, 0, st>>>(X, ldx, mu, sigma, row0, n_units, D, key, stream_off, f, pa.sink,
-                                                                                pa.epoch, pa.done);
+    auto k = sample_eval_kernel<OBJ, SYM, STORE, false>;
+    k<<<resident_grid(k, kSampleThreads, ctas_needed), kSampleThreads, 0, st>>>(X, ldx, mu, sigma, row0, n_units, D, key, stream_off, f);
   }
   EVOK_CHECK_LAUNCH();
   return 0;
@@ -239,17 +217,6 @@ static int dispatch_sample(float* X, int64_t ldx, const float* mu, const float* 
   }
   return X ? launch_sample<OBJ, false, true>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, f, st)
            : launch_sample<OBJ, false, false>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, f, st);
-}
-
-template <int OBJ>
-static int dispatch_sample_push(float* X, int64_t ldx, const float* mu, const float* sigma, int64_t row0, int64_t n_rows, int64_t D,
-                                int symmetric, uint64_t seed, uint64_t stream_id, const uint32_t* stream_off, const PushArgs& push, cudaStream_t st) {
-  if (symmetric) {
-    return X ? launch_sample<OBJ, true, true, true>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, nullptr, st, &push)
-             : launch_sample<OBJ, true, false, true>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, nullptr, st, &push);
-  }
-  return X ? launch_sample<OBJ, false, true, true>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, nullptr, st, &push)
-           : launch_sample<OBJ, false, false, true>(X, ldx, mu, sigma, row0, n_rows, D, seed, stream_id, stream_off, nullptr, st, &push);
 }
 
 template <int OBJ>
@@ -288,35 +255,6 @@ extern "C" EVOK_API int evok_sample_eval(int objective, float* X, int64_t ldx, c
     case EVOK_OBJ_SPHERE: return dispatch_sample<EVOK_OBJ_SPHERE>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_off, f, st);
     case EVOK_OBJ_RASTRIGIN: return dispatch_sample<EVOK_OBJ_RASTRIGIN>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_off, f, st);
     case EVOK_OBJ_ACKLEY: return dispatch_sample<EVOK_OBJ_ACKLEY>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_off, f, st);
-  }
-  return EVOK_E_BADENUM;
-}
-
-extern "C" EVOK_API int evok_sample_eval_push(int objective, float* X, int64_t ldx, const float* mu, const float* sigma, int64_t row0, int64_t n_rows,
-                                              int64_t D, int symmetric, uint64_t seed, uint64_t stream_id, const uint32_t* stream_offset_dev,
-                                              int world, int rank, void* const* peer_f, void* const* peer_flags, const uint64_t* epoch_dev,
-                                              uint32_t* done_dev, void* stream) {
-  if (!mu || !sigma || !peer_f || !peer_flags || !epoch_dev || !done_dev) return EVOK_E_NULLPTR;
-  if (objective <= EVOK_OBJ_NONE || objective >= EVOK_OBJ_COUNT) return EVOK_E_BADENUM;
-  if (world < 1 || world > EVOK_MAX_PEERS || rank < 0 || rank >= world) return EVOK_E_BADSIZE;
-  if (n_rows < 0 || D <= 0 || row0 < 0 || (X && ldx < D)) return EVOK_E_BADSIZE;
-  if (symmetric && ((n_rows & 1) || (row0 & 1))) return EVOK_E_ODDROWS;
-  PushArgs push{};
-  push.sink.world = world;
-  push.sink.rank = rank;
-  for (int p = 0; p < world; ++p) {
-    if (!peer_f[p] || !peer_flags[p]) return EVOK_E_NULLPTR;
-    push.sink.data[p] = peer_f[p];
-    push.sink.flags[p] = static_cast<unsigned long long*>(peer_flags[p]);
-  }
-  push.epoch = reinterpret_cast<const unsigned long long*>(epoch_dev);
-  push.done = done_dev;
-  // n_rows == 0 still launches one CTA: the peers wait for this rank's flag
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (objective) {
-    case EVOK_OBJ_SPHERE: return dispatch_sample_push<EVOK_OBJ_SPHERE>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_offset_dev, push, st);
-    case EVOK_OBJ_RASTRIGIN: return dispatch_sample_push<EVOK_OBJ_RASTRIGIN>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_offset_dev, push, st);
-    case EVOK_OBJ_ACKLEY: return dispatch_sample_push<EVOK_OBJ_ACKLEY>(X, ldx, mu, sigma, row0, n_rows, D, symmetric, seed, stream_id, stream_offset_dev, push, st);
   }
   return EVOK_E_BADENUM;
 }

@@ -170,16 +170,11 @@ def sharded_sample_and_gradients(problem, distribution, popsize: int, *, obj_ind
     # sharded ranking: sort locally, exchange sorted keys, rank the local rows against the world (no GPU holds all fitnesses)
     sharded_rank = (peer is not None and method in ("centered", "linear", "nes") and dev_dist.accepts_local_weights(method)
                     and os.environ.get("EVOTORCH_B200_SHARDED_RANK", "0") == "1")  # opt-in: measured equal to the replicated sort at 8 GPUs
-    # the fitness all-gather: either stores from inside the sampler (EVOTORCH_B200_PUSH_IN_SAMPLER=1, the round-1 protocol) or, by
-    # default, the plain sampler followed by one 8-CTA push kernel (coalesced 16-byte stores, one system fence per peer)
-    push_in_sampler = peer is not None and not sharded_rank and os.environ.get("EVOTORCH_B200_PUSH_IN_SAMPLER", "0") == "1"
     problem.philox_row0 = row0
-    problem._active_peer = peer if push_in_sampler else None  # otherwise the fitnesses are written locally by the plain fused sampler
     try:
         problem.sample_and_evaluate(dev_dist, batch)
     finally:
         problem.philox_row0 = 0
-        problem._active_peer = None
 
     samples = batch.recipe if isinstance(batch, LazySolutionBatch) else batch.access_values(keep_evals=True)
     if sharded_rank:
@@ -201,8 +196,9 @@ def sharded_sample_and_gradients(problem, distribution, popsize: int, *, obj_ind
         grads, mean_eval = _results_to_home(problem, grads, mean_eval, home_device)
         return {"gradients": grads, "num_solutions": popsize, "mean_eval": mean_eval}
     if peer is not None:
-        if not push_in_sampler:
-            peer.push_fitness(row0, n_local)
+        # the fitness all-gather: the sampler wrote this rank's slice of f_all locally; one push kernel copies it to every peer
+        # (coalesced 16-byte stores, one system fence per peer)
+        peer.push_fitness(row0, n_local)
         f_all = peer.wait_fitness()
     else:
         f_local = batch.access_evals(obj_index)

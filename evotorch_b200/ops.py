@@ -135,27 +135,6 @@ def sample_eval(objective: int, X: Optional[torch.Tensor], mu: torch.Tensor, sig
     nat.check(rc, "evok_sample_eval")
 
 
-def sample_eval_push(objective: int, X: Optional[torch.Tensor], mu: torch.Tensor, sigma: torch.Tensor, *, n_rows: int, symmetric: bool,
-                     seed: int, stream_id: int, row0: int, peer, stream_offset: Optional[torch.Tensor] = None) -> None:
-    """K1+K2 with the fitness all-gather fused in: row i's fitness lands in `f_all[row0 + i]` of every rank (`peer` is a
-    evotorch_b200.peer.PeerExchange).  Follow with `peer.wait_fitness()` before reading `peer.f_all`."""
-    D = mu.numel()
-    _vec(mu, "mu"); _vec(sigma, "sigma", D)
-    ldx = 0
-    if X is not None:
-        _mat(X, "X")
-        if X.shape != (n_rows, D):
-            raise ValueError(f"X: expected shape {(n_rows, D)}, got {tuple(X.shape)}")
-        ldx = X.stride(0)
-    if row0 + n_rows > peer.popsize:
-        raise ValueError("rows beyond the population the peer exchange was sized for")
-    with _timed("sample_eval"):
-        rc = nat.lib().evok_sample_eval_push(objective, nat.ptr(X), ldx, mu.data_ptr(), sigma.data_ptr(), row0, n_rows, D, int(symmetric),
-                                             seed & 0xFFFFFFFFFFFFFFFF, stream_id & 0xFFFFFFFFFFFFFFFF, _offset_ptr(stream_offset), peer.world,
-                                             peer.rank, peer.peer_f, peer.peer_flags_f, peer.epoch_f, peer._counter(0), nat.stream_of(mu))
-    nat.check(rc, "evok_sample_eval_push")
-
-
 def grad_push(form: int, X: Optional[torch.Tensor], w: torch.Tensor, mu: torch.Tensor, sigma: torch.Tensor, *, scale_mu: float,
               scale_sigma: float, peer, seed: int = 0, stream_id: int = 0, row0: int = 0, stream_offset: Optional[torch.Tensor] = None) -> None:
     """K4 with the send half of the gradient all-reduce fused in (X = None: regenerate the rows from the Philox counters).

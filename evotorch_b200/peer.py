@@ -1,9 +1,10 @@
-"""Peer exchange: the two collectives of the sharded generation done by the producing kernels themselves over NVLink.
+"""Peer exchange: the two collectives of the sharded generation done by libevok kernels over NVLink.
 
 `torch.distributed` (NCCL) stays the control plane -- it carries the 64-byte IPC handles once, at set-up.  After that a
 generation contains no library collective at all:
 
-  K1+K2  sample_eval_kernel<PUSH>      stores each fitness into EVERY peer's fitness vector; last CTA raises the flags
+  K1+K2  sample_eval_kernel             writes this rank's fitness slice into its local copy of the fitness vector
+         peer_push_kernel               copies the slice into EVERY peer's fitness vector and raises the flags
          peer_wait_kernel               one warp waits for all ranks' flags                         (was: all_gather)
   K3     rank (replicated, on the local copy of the full fitness vector)
   K4     grad_partial + grad_finalize_push_kernel   this rank's (grad_mu | grad_sigma) -> slot[rank] on every peer + flags
@@ -91,7 +92,8 @@ class PeerExchange:
         self.f_all = _view(self._base + self._off_f, n, "<f4", self.device)
         self.slots = _view(self._base + self._off_slots, r * 2 * d, "<f4", self.device)
         self._flags_f_ptr, self._flags_g_ptr = self._base + self._off_flags_f, self._base + self._off_flags_g
-        # local (unshared) state: [epoch_f, epoch_g] u64, [done_f, done_g, done_r, err] u32
+        # local (unshared) state: [epoch_f, epoch_g] u64, [done_f, done_g, done_r, err] u32 (done_f is unused: the fitness push
+        # kernel raises the flags from its own per-peer CTA and needs no completion counter)
         self._epochs = torch.zeros(2, dtype=torch.int64, device=self.device)
         self._counters = torch.zeros(4, dtype=torch.int32, device=self.device)
         self._rank_counters = torch.zeros(4, dtype=torch.int32, device=self.device)  # sharded ranking: hist-scan / push / merge

@@ -208,24 +208,13 @@ int evok_mlp_forward_prep(const float* params, int64_t ldp, const float* obs, in
 /* The forward of N networks on ONE shared input batch (B x dims[0]) -- a population scored on a common minibatch
  * (neuroevolution/supervisedne.py:337-347, where the reference loops over the solutions: parameterize_net + network(x), neproblem.py:342,
  * supervisedne.py:250).  Here the first layer of ALL networks is one tensor-core product of the stacked weight rows with the shared batch
- * (evok_gemm_gather_rows: the weight rows are gathered from the flat parameter rows -- any 4-byte alignment -- straight into the swizzled
+ * (a persistent kernel gathers the weight rows from the flat parameter rows -- any 4-byte alignment -- straight into the swizzled
  * operand tiles, so every parameter is read from HBM once; bias and activation in the epilogue), the remaining (small, per-network)
  * layers run in a second kernel on the staged activations.  out: [N][B][dims[n_layers]].  n_layers >= 2, hidden widths <= 512,
  * X 16-byte aligned with ldx % 4 == 0. */
 size_t evok_mlp_forward_shared_workspace_bytes(int64_t N, int64_t B, int n_layers, const int32_t* dims_host);
 int evok_mlp_forward_shared(const float* params, int64_t ldp, int64_t N, const float* X, int64_t ldx, int64_t B, int n_layers,
                             const int32_t* dims_host, const int32_t* acts_host, float* out, void* ws, size_t ws_bytes, void* stream);
-/* C[(i, h), b] = act(sum_k W_i[h, k] X[b, k] + bias_i[h]),  W_i = params + i * batch_stride + w_offset (rows_per_batch x K, row-major),
- * bias_i = params + i * batch_stride + bias_offset (bias_offset < 0: none).  3xTF32 on tcgen05, fp32 accuracy. */
-int evok_gemm_gather_rows(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch, int64_t n_batches, const float* X,
-                          int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset, int act, float* C, int64_t ldc, void* stream);
-/* The same product on the PERSISTENT kernel (one CTA per SM walks the tiles; X pre-split into hi / lo copies in `ws`, so X may have any
- * alignment; epilogue overlapped with the next tile).  unit_fastest != 0: C[(batch * n_cols + col) * rows_per_batch + row] (ldc unused)
- * instead of C[(batch * rows_per_batch + row) * ldc + col].  Used by evok_mlp_forward_shared. */
-size_t evok_gemm_gather_rows_workspace_bytes(int64_t n_cols, int64_t K);
-int evok_gemm_gather_rows_ws(const float* params, int64_t batch_stride, int64_t w_offset, int64_t rows_per_batch, int64_t n_batches, const float* X,
-                             int64_t ldx, int64_t n_cols, int64_t K, int64_t bias_offset, int act, float* C, int64_t ldc, int unit_fastest, void* ws,
-                             size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K6 / K7: fp32-accurate tensor-core GEMM (tcgen05 + TMEM + TMA, 3xTF32 operand splitting).
@@ -303,14 +292,14 @@ int evok_cholesky(const float* A, int64_t lda, int64_t n, float* L, int64_t ldl,
 
 /* ---------------------------------------------------------------------------------------------
  * Peer exchange over NVLink / NVSwitch: the two collectives of the sharded generation (the reference's Ray round trip,
- * core.py:2762-3073 + algorithms/distributed/gaussian.py:199-272; evotorch_b200/distributed.py) fused into their
- * producing kernels.  One process per GPU; every rank owns one "exchange buffer" that all peers map (CUDA IPC).
+ * core.py:2762-3073 + algorithms/distributed/gaussian.py:199-272; evotorch_b200/distributed.py) done by libevok kernels.
+ * One process per GPU; every rank owns one "exchange buffer" that all peers map (CUDA IPC).  The *_host tables are host
+ * arrays of `world` device pointers, one per peer; peer_flags_host[p] = base of peer p's `world` 64-bit flags.
  *
  *   evok_peer_alloc / open / close / free : the only entry points that allocate.  `handle` is a 64-byte cudaIpcMemHandle_t
  *       to be passed to the other processes (any transport).  The buffer is zero-filled.
- *   evok_sample_eval_push : evok_sample_eval whose fitness store goes to row (row0 + i) of EVERY peer's fitness vector
- *       (peer_f_host[p] = base of peer p's N-float vector; the *_host tables are host arrays of `world` device pointers) -- the all-gather.  The last CTA raises flag[rank] = *epoch_dev + 1 in
- *       every peer's flag array (peer_flags_host[p] = base of peer p's `world` 64-bit flags).
+ *   evok_peer_push : the all-gather.  Runs behind the producer (evok_sample_eval into this rank's slice of the local fitness
+ *       vector) and copies that slice to every peer, then raises flag[rank] = *epoch_dev + 1 in every peer's flag array.
  *   evok_peer_wait : one warp spins until all `world` local flags reach *epoch_dev + 1, then advances *epoch_dev.  After
  *       `timeout_ns` it gives up, sets *err_dev = 1 and advances anyway (no hang; the host checks err_dev when it likes).
  *   evok_grad_push : evok_grad / evok_grad_regen (X == NULL) whose finalisation writes this rank's (grad_mu | grad_sigma)
@@ -339,13 +328,9 @@ int evok_peer_alloc(size_t bytes, void** dev_ptr_out_host, void* handle_out_64B_
 int evok_peer_open(const void* handle_64B_host, void** dev_ptr_out_host);
 int evok_peer_close(void* dev_ptr);
 int evok_peer_free(void* dev_ptr);
-int evok_sample_eval_push(int objective, float* X, int64_t ldx, const float* mu, const float* sigma, int64_t row0, int64_t n_rows,
-                          int64_t D, int symmetric, uint64_t seed, uint64_t stream_id, const uint32_t* stream_offset_dev, int world,
-                          int rank, void* const* peer_f_host, void* const* peer_flags_host, const uint64_t* epoch_dev, uint32_t* done_dev,
-                          void* stream);
 /* evok_peer_push: the all-gather as ONE small kernel behind the producer: CTA p copies this rank's slice (n_bytes at src_local) to
  * offset dst_offset_bytes of peer p's buffer (peer_base_host[p]) with 16-byte stores, fences once and raises flag[rank] = *epoch_dev + 1
- * on that peer.  Consumer: evok_peer_wait, as for evok_sample_eval_push. */
+ * on that peer.  Consumer: evok_peer_wait. */
 int evok_peer_push(const void* src_local, int64_t n_bytes, int64_t dst_offset_bytes, int world, int rank, void* const* peer_base_host,
                    void* const* peer_flags_host, const uint64_t* epoch_dev, void* stream);
 int evok_peer_wait(const uint64_t* flags_local, int world, uint64_t* epoch_dev, uint32_t* err_dev, uint64_t timeout_ns, void* stream);

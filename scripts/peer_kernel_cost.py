@@ -1,4 +1,5 @@
-"""Single GPU, world size 1: cost of the push variants of the producers vs the plain kernels (same work, plus flag traffic)."""
+"""Single GPU, world size 1: cost of the peer-exchange path of the producers (plain sampler + push kernel + wait, gradient push +
+reduce) vs the plain kernels (same work, plus flag traffic)."""
 import os
 import sys
 import tempfile
@@ -39,7 +40,8 @@ def plain_sample():
 
 
 def push_sample():
-    ops.sample_eval_push(ops.OBJ_RASTRIGIN, X, mu, sigma, n_rows=n, symmetric=True, seed=1, stream_id=5, row0=0, peer=px)
+    ops.sample_eval(ops.OBJ_RASTRIGIN, X, mu, sigma, n_rows=n, symmetric=True, seed=1, stream_id=5, f=px.f_all)
+    px.push_fitness(0, n)
     px.wait_fitness()
 
 

@@ -91,7 +91,8 @@ px = PeerExchange(n, D, torch.device(dev), timeout_ns=2_000_000_000)
 mu, sg = torch.randn(D, device=dev), torch.rand(D, device=dev) + 0.1
 X = torch.empty(n, D, device=dev)
 for gen in range(3):
-    ops.sample_eval_push(2, X, mu, sg, n_rows=n, symmetric=True, seed=3, stream_id=gen, row0=0, peer=px)
+    ops.sample_eval(2, X, mu, sg, n_rows=n, symmetric=True, seed=3, stream_id=gen, f=px.f_all[0:n])
+    px.push_fitness(0, n)
     w = ops.rank(px.wait_fitness(), "centered", False)
     ops.grad_push(ops.GRAD_SYMMETRIC, X, w, mu, sg, scale_mu=1.0, scale_sigma=1.0, peer=px)
     px.reduce_gradients()
@@ -99,9 +100,6 @@ for gen in range(3):
     px.reduce_gradients()
 assert not px.timed_out()
 # ---- round-2 kernels
-# peer push / sharded ranking on one rank (local "peers")
-px.push_fitness(0, n)
-px.wait_fitness()
 # shared-minibatch policy forward: persistent gather GEMM (16-byte path at every row alignment, 4-byte path, generic tail) + tail kernels
 from evotorch_b200.neuroevolution import Policy  # noqa: E402
 

@@ -788,9 +788,9 @@ def single_rank_group(tmp_path):
     dist.destroy_process_group()
 
 
-def test_peer_exchange_kernels_single_rank(single_rank_group):
-    """World size 1 runs the very same kernels as the multi-GPU exchange (push stores + flag raise, flag wait, slot
-    reduction); the results must equal the plain kernels bit for bit, generation after generation, also from a CUDA graph.
+def test_peer_exchange_push_kernel_single_rank(single_rank_group):
+    """World size 1 runs the very same kernels as the multi-GPU exchange (fitness push + flag raise, flag wait, gradient push,
+    slot reduction); the results must equal the plain kernels bit for bit, generation after generation, also from a CUDA graph.
     (2- and 8-GPU parity: scripts/check_peer_exchange.py, profiles/r01_peer_exchange_*.txt.)"""
     from evotorch_b200.peer import PeerExchange
 
@@ -803,7 +803,8 @@ def test_peer_exchange_kernels_single_rank(single_rank_group):
     f = torch.empty(n, device=DEV)
 
     def generation(gen):
-        ops.sample_eval_push(ops.OBJ_RASTRIGIN, Xp, mu, sigma, n_rows=n, symmetric=True, seed=9, stream_id=gen, row0=0, peer=px)
+        ops.sample_eval(ops.OBJ_RASTRIGIN, Xp, mu, sigma, n_rows=n, symmetric=True, seed=9, stream_id=gen, f=px.f_all[0:n])
+        px.push_fitness(0, n)
         f_all = px.wait_fitness()
         w = ops.rank(f_all, "centered", False)
         ops.grad_push(ops.GRAD_SYMMETRIC, Xp, w, mu, sigma, scale_mu=2.0 / n, scale_sigma=2.0 / n, peer=px)
@@ -834,14 +835,6 @@ def test_peer_exchange_kernels_single_rank(single_rank_group):
     torch.testing.assert_close(out[0], rmu, rtol=0, atol=2e-6)
     torch.testing.assert_close(out[1], rsig, rtol=0, atol=2e-6)
     assert px._epochs.tolist() == [3, 7] and not px.timed_out()
-    # round 2: the plain sampler writing the local slice + ONE push kernel (evok_peer_push) instead of stores from inside the sampler
-    for gen in range(3, 5):
-        ops.sample_eval(ops.OBJ_RASTRIGIN, Xp, mu, sigma, n_rows=n, symmetric=True, seed=9, stream_id=gen, f=px.f_all[0:n])
-        px.push_fitness(0, n)
-        f_all = px.wait_fitness()
-        ops.sample_eval(ops.OBJ_RASTRIGIN, X, mu, sigma, n_rows=n, symmetric=True, seed=9, stream_id=gen, f=f)
-        assert torch.equal(f, f_all), gen
-    assert px._epochs.tolist() == [5, 7] and not px.timed_out()
     px.close()
 
 
